@@ -15,6 +15,16 @@ enable_tma=False, autotuned; fetched into the git-ignored baseline/_ref/ by scri
 seeded inputs with the same CUDA-event method: the GPU comparator the north-star names.
 `--impl reference` times the CPU port of the reference eager path (oracle/) on the host cores on a bounded sample of
 the same workload (the Python reference itself cannot travel to the GPU box).  Rank 0 only.
+
+`--dump-outputs DIR` (GPU workloads) writes, after the timed steps, what the last step returned to its caller as
+DIR/<name>.npy in float32 (at most 64 MB in all; row-sampled with a fixed seed where an output is larger), so that two builds
+can be compared output for output on identical seeded inputs.  Two runs of the same build do not agree bit for bit: the
+attention backward's dQ accumulation order varies (2e-5 relative), and AdamW on bf16 weights amplifies that over the steps.
+Measured on one B200 (1000 W power limit), default workload, rel-L2 between two runs: after 3 steps up to 1.1e-2 on y and
+5e-3 on the parameter gradients; the loss agrees to 2e-6.
+
+bench.py writes nothing into the source tree: it loads the library that `python -m generative_recommenders_b200.build`
+(or __graft_entry__.build()) left there and does not compile.
 """
 import argparse
 import json
@@ -28,6 +38,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 
@@ -48,7 +59,14 @@ def parse_args():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: --batch sequences per GPU (default, what the driver's scaling run measures); strong: --batch "
                          "sequences in total, sharded over the ranks balanced by sum(len^2) (distributed.shard_sequences)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last step as DIR/<name>.npy (float32, <= 64 MB in all)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -142,6 +160,33 @@ def attn_inputs(L, heads, d, dev):
     return x, do
 
 
+DUMP_BYTES = 64_000_000  # all files of --dump-outputs together
+DUMP_SEED = 12345  # row sample of outputs that do not fit whole
+
+
+def dump_outputs(out_dir, whole, sampled):
+    """Write every tensor of `whole` entirely and of every tensor of `sampled` a seeded sample of rows (dim 0), as many as
+    the rest of DUMP_BYTES allows, as out_dir/<name>.npy in float32.  The sample depends only on the row count and
+    DUMP_SEED, so two runs with the same arguments write the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {name: t.detach().float().cpu() for name, t in whole.items()}
+    header = 128  # .npy header of one file (format 1.0)
+    left = DUMP_BYTES - sum(a.numel() * 4 + header for a in arrays.values()) - header * len(sampled)
+    for name, t in sampled.items():
+        rows = t.shape[0]
+        row_bytes = 4 * (t.numel() // max(rows, 1))
+        keep = min(rows, max(0, left // len(sampled)) // max(row_bytes, 1))
+        idx = torch.randperm(rows, generator=torch.Generator().manual_seed(DUMP_SEED))[:keep].sort().values
+        arrays[name] = t.detach()[idx.to(t.device)].float().cpu()
+    total = 0
+    for name, a in arrays.items():
+        path = os.path.join(out_dir, f"{name}.npy")
+        np.save(path, a.numpy())
+        total += os.path.getsize(path)
+    assert total <= DUMP_BYTES, (total, DUMP_BYTES)
+    return total
+
+
 def attn_flops(lengths, heads, dqk, dv):
     """Reference FLOP model (hstu_attention_bench.py:35-59): causal-halved, 2 FLOP per MAC."""
     s2 = float((lengths.double() ** 2).sum())
@@ -162,7 +207,6 @@ def attn_bytes(lengths, heads, dqk, dv, elt=2):
 def run_ours(args):
     import torch.distributed as dist
     from generative_recommenders_b200 import _lib
-    from generative_recommenders_b200.build import build
     from generative_recommenders_b200.modules.stu import STULayer, STULayerConfig, STUStack
     from generative_recommenders_b200.ops.hstu_attention import hstu_mha
 
@@ -173,8 +217,7 @@ def run_ours(args):
         raise SystemExit("bench.py needs a CUDA device: the product path has no CPU fallback")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
-    if rank == 0:
-        build()
+    last = {} if args.dump_outputs and rank == 0 else None  # outputs of the latest step, for --dump-outputs
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
         dist.barrier()
@@ -231,6 +274,8 @@ def run_ours(args):
             loss.backward()
             reducer.wait()
             opt.step()
+            if last is not None:
+                last["y"], last["loss"] = y, loss
             if e2e:
                 return float(loss.item())  # device -> host read of the step result
             return loss
@@ -266,6 +311,8 @@ def run_ours(args):
                 q.grad = k.grad = v.grad = None
             o = hstu_mha(args.lmax, alpha, qq, kk, vv, off, num_targets=nt, sort_by_length=True, impl=args.attn_impl)
             o.backward(do)
+            if last is not None:
+                last.update(out=o, dq=qq.grad, dk=kk.grad, dv=vv.grad)
             if e2e:
                 return float(o[0, 0, 0].item())
             return o
@@ -315,6 +362,14 @@ def run_ours(args):
     ms, launches, events = timed_run(False, args.steps, args.warmup, True)
     clocks = sampler.stop() if sampler else None
     ms_e2e, _, _ = timed_run(True, args.steps, 1, False)
+    if last is not None:
+        if args.workload == "hstu_large":
+            # the training step returns the loss and leaves the stack output and the parameter gradients to its caller
+            whole = {"loss": last["loss"]}
+            whole.update({f"grad.{n}": p.grad for n, p in stack.named_parameters()})
+            dump_outputs(args.dump_outputs, whole, {"y": last["y"]})
+        else:
+            dump_outputs(args.dump_outputs, {}, {k: last[k] for k in ("out", "dq", "dk", "dv")})
 
     value = units_per_step * world * args.steps / (ms * 1e-3)
     value_e2e = units_per_step * world * args.steps / (ms_e2e * 1e-3)
@@ -375,7 +430,6 @@ RESEARCH_CFG = {
 
 def run_research(args):
     from generative_recommenders_b200 import _lib
-    from generative_recommenders_b200.build import build
     from generative_recommenders_b200.modules.research_hstu import (RelativeBucketedTimeAndPositionBasedBias,
                                                                     SequentialTransductionUnitJagged)
     from generative_recommenders_b200.modules.sampled_softmax import LocalNegativesSampler, SampledSoftmaxLoss
@@ -383,7 +437,6 @@ def run_research(args):
     c = RESEARCH_CFG[args.workload]
     dev = torch.device("cuda", int(os.environ.get("LOCAL_RANK", "0")))
     torch.cuda.set_device(dev)
-    build()
     _lib.lib()
     torch.manual_seed(7)
     D, H, d, n, B, R, V = c["D"], c["H"], c["d"], c["n"], c["B"], c["R"], c["V"]
@@ -410,6 +463,7 @@ def run_research(args):
     ids_dev, ts_dev = ids_host.to(dev), ts_host.to(dev)
     nxt = torch.arange(1, L + 1, device=dev).clamp(max=L - 1)  # next-item supervision inside the flat row order (synthetic)
     w_dev = torch.ones(L, device=dev, dtype=torch.bfloat16)
+    last = {} if args.dump_outputs else None  # outputs of the latest step, for --dump-outputs
 
     def step(e2e):
         ids = ids_host.to(dev, non_blocking=True) if e2e else ids_dev
@@ -423,6 +477,8 @@ def run_research(args):
                                           supervision_weights=w_dev, negatives_sampler=sampler)
         loss.backward()
         opt.step()
+        if last is not None:
+            last["x"], last["loss"] = x, loss
         return float(loss.item()) if e2e else loss
 
     def timed(e2e, steps, warmup, with_events):
@@ -446,6 +502,12 @@ def run_research(args):
     ms, launches, events = timed(False, args.steps, args.warmup, True)
     clocks = sampler_c.stop()
     ms_e2e, _, _ = timed(True, args.steps, 1, False)
+    if last is not None:
+        # the loss, the output embeddings of the last block and the gradients of the blocks; the item table's gradient (V x D)
+        # is row-sampled like the embeddings
+        whole = {"loss": last["loss"]}
+        whole.update({f"grad.{n}": p.grad for n, p in model["blocks"].named_parameters() if p.grad is not None})
+        dump_outputs(args.dump_outputs, whole, {"x": last["x"], "grad.emb.weight": model["emb"].weight.grad})
     kt = {k: round(sum(a.elapsed_time(b) for a, b in v) / max(1, len(v)), 4) for k, v in (events or {}).items()}
     print(json.dumps({
         "metric": f"user-seqs/sec {c['name']} (research path) fwd+bwd+AdamW", "value": B * args.steps / (ms * 1e-3), "unit": "sequences/s",
@@ -727,6 +789,7 @@ def run_reference(args):
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ next to the sources
     a = parse_args()
     if a.impl == "reference":
         run_reference(a)

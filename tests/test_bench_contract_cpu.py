@@ -54,6 +54,26 @@ def test_traffic_is_reported_only_for_the_captured_shape():
     assert b.ncu_traffic({"attn_shape": other}) == (None, None)
 
 
+def test_dump_outputs_fits_the_budget_and_samples_the_same_rows(tmp_path):
+    import numpy as np
+    import torch
+
+    b = _bench()
+    whole = {"loss": torch.tensor(0.25), "grad.w": torch.randn(3000, 1024)}
+    big = torch.randn(100_000, 256, dtype=torch.bfloat16)  # 102 MB as float32: must be row-sampled
+    for run in ("a", "b"):
+        b.dump_outputs(str(tmp_path / run), whole, {"y": big})
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["grad.w.npy", "loss.npy", "y.npy"]
+    assert sum((tmp_path / "a" / f).stat().st_size for f in files) <= b.DUMP_BYTES
+    for f in files:
+        a, c = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float32 and np.array_equal(a, c)
+    y = np.load(tmp_path / "a" / "y.npy")
+    assert 10_000 < y.shape[0] < big.shape[0] and y.shape[1] == 256
+    assert np.array_equal(np.load(tmp_path / "a" / "grad.w.npy"), whole["grad.w"].numpy())
+
+
 def test_round2_lines():
     one, two, strong = _load("r02_bench_1gpu.json"), _load("r02_bench_2gpu.json"), _load("r02_bench_2gpu_strong.json")
     for d, n, scaling in ((one, 1, "weak"), (two, 2, "weak"), (strong, 2, "strong")):
